@@ -74,6 +74,11 @@ def parse_args():
                     help="replay the training step from a CUDA graph (core.StepGraph). auto = on for "
                          "single-GPU dlrm and the launch-bound workloads (fm, din, autoint, youtubednn), "
                          "off for sasrec and for multi-GPU runs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the loss of the last one and the model parameters "
+                         "and buffers it left (large embedding tables as a fixed sample of updated rows; "
+                         "no optimizer state) to DIR/<name>.npy, so that two builds can be compared "
+                         "output for output (single process only)")
     return ap.parse_args()
 
 
@@ -83,6 +88,56 @@ def load_peaks():
         with open(path) as f:
             return json.load(f), "measured (MEASURED_PEAKS.json)"
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0}, "fallback (B200_PROFILING.md)"
+
+
+DUMP_ROWS = 512                 # rows kept of a table larger than DUMP_TABLE_ROWS
+DUMP_TABLE_ROWS = 4096
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, loss, model):
+    """--dump-outputs: `loss` (what the last timed step returned) and the parameters and buffers
+    that step left in `model`, one DIR/<name>.npy per float tensor (float64 stays float64, the rest
+    is written as float32).  Optimizer state (Adam moments) is not written.  Of a 2-D tensor with
+    more than DUMP_TABLE_ROWS rows (an embedding table) only DUMP_ROWS rows are kept, listed in
+    DIR/<name>.rows.npy and drawn with a fixed seed among the rows the table's sparse optimizer has
+    updated (non-zero first moment), so that they carry what training computed; a table without
+    optimizer state is sampled over all its rows."""
+    import zlib
+
+    import numpy as np
+    import torch
+    from recommend_tf2_b200.embedding import EmbeddingTables
+    params = dict(model.named_parameters())
+    updated = {}
+    for mname, mod in model.named_modules():
+        if isinstance(mod, EmbeddingTables):
+            for i, m1 in enumerate(mod.state1):
+                if m1 is not None:
+                    updated[f"{mname}.weights.{i}".lstrip(".")] = m1.ne(0).any(1).nonzero()[:, 0]
+    if not set(updated) <= set(params):
+        raise RuntimeError(f"--dump-outputs: tables {sorted(set(updated) - set(params))} not among the "
+                           "model's parameters")
+    out = {"loss": loss}
+    for name, t in list(params.items()) + list(model.named_buffers()):
+        if not t.is_floating_point():
+            continue
+        if t.dim() == 2 and t.shape[0] > DUMP_TABLE_ROWS:
+            rng = np.random.default_rng(zlib.crc32(name.encode()))
+            cand = updated[name].cpu().numpy() if len(updated.get(name, ())) else np.arange(t.shape[0])
+            rows = np.sort(cand[rng.choice(len(cand), min(DUMP_ROWS, len(cand)), replace=False)])
+            rows = torch.from_numpy(rows).long()
+            out[name + ".rows"] = rows.double()
+            t = t[rows.to(t.device)]
+        out[name] = t
+    arrays = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32).numpy()
+              for k, v in out.items()}
+    nbytes = sum(v.nbytes for v in arrays.values())
+    if nbytes > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {nbytes} bytes (limit {DUMP_MAX_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def make_batches(n, B, rows, ids_kind, seed):
@@ -428,6 +483,9 @@ def run_b200(args):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     torch.backends.cuda.matmul.allow_tf32 = False   # fp32 parity with the reference (1e-5)
     torch.backends.cudnn.allow_tf32 = False
+    # the MLP weights come from torch's default CUDA generator, which torch seeds at random in every
+    # process: seeded here, runs with the same arguments start from the same model
+    torch.manual_seed(1234)
 
     import recommend_tf2_b200 as pkg
     pkg.lib()
@@ -508,13 +566,15 @@ def run_b200(args):
     t_start = time.time()
     e0.record()
     for i in range(W, W + K):
-        trainer.step(*dev[i], **nxt(i))
+        last_loss = trainer.step(*dev[i], **nxt(i))
     e1.record()
     host_ms = (time.time() - t_start) * 1e3 / K     # host enqueue time (the CPU runs ahead of the GPU)
     barrier()
     t_end = time.time()
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop(t_start, t_end) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_loss, model)
 
     # ---- end to end: pinned host batches in, loss out, every step, inside the timed region
     loss_host = torch.zeros(K, dtype=torch.float32).pin_memory()
@@ -667,6 +727,7 @@ def run_workload(args):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     torch.backends.cuda.matmul.allow_tf32 = False
     torch.backends.cudnn.allow_tf32 = False
+    torch.manual_seed(1234)     # same model from run to run (see run_b200)
     import recommend_tf2_b200 as pkg
     pkg.lib()
     peaks, peak_src = load_peaks()
@@ -699,12 +760,14 @@ def run_workload(args):
     t_start = time.time()
     e0.record()
     for i in range(W, W + K):
-        st.step(*dev[i])
+        last_loss = st.step(*dev[i])
     e1.record()
     barrier()
     t_end = time.time()
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop(t_start, t_end) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_loss, st.model)
 
     loss_host = torch.zeros(K, dtype=torch.float32).pin_memory()
     for _ in pkg.DeviceFeeder(host[:2]):
@@ -770,6 +833,8 @@ class _StepShim:
 
 def main():
     args = parse_args()
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        raise SystemExit("bench.py: --dump-outputs runs in a single process (--gpus 1)")
     if args.workload != "dlrm":
         return run_workload_reference(args) if args.impl == "reference" else run_workload(args)
     if args.replicate_max_rows < 0:     # same resolved config for both arms

@@ -37,6 +37,37 @@ def test_b200_arm_refuses_to_run_without_cuda():
     assert "no CUDA device" in (res.stderr + res.stdout)
 
 
+def test_dump_outputs_writes_loss_state_and_sampled_table_rows(tmp_path):
+    """--dump-outputs: the loss, every float parameter / buffer as .npy (float64 kept, the rest
+    float32), tables above DUMP_TABLE_ROWS rows as a seeded sample of the rows their sparse
+    optimizer has updated (all rows without optimizer state), the same files for the same state."""
+    import numpy as np
+    import torch
+    import bench
+    from recommend_tf2_b200.embedding import EmbeddingTables, SparseOptimizer
+
+    n = bench.DUMP_TABLE_ROWS + 1000
+    m = torch.nn.Module()
+    m.emb = EmbeddingTables([n, 50], [4, 4], device="cpu", optimizer=SparseOptimizer("adam"))
+    m.plain = EmbeddingTables([n], [4], device="cpu")
+    m.dense = torch.nn.Linear(4, 3).double()
+    updated = torch.randperm(n)[:3000]
+    m.emb.state1[0][updated] = 1e-3
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), torch.tensor(0.25, dtype=torch.bfloat16), m)
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert sorted(got) == ["dense.bias", "dense.weight", "emb.weights.0", "emb.weights.0.rows", "emb.weights.1",
+                           "loss", "plain.weights.0", "plain.weights.0.rows"]
+    assert got["loss"] == 0.25 and got["loss"].dtype == np.float32 and got["dense.weight"].dtype == np.float64
+    rows = got["emb.weights.0.rows"].astype(np.int64)
+    assert len(rows) == bench.DUMP_ROWS and np.isin(rows, updated.numpy()).all()
+    np.testing.assert_array_equal(got["emb.weights.0"], m.emb.weights[0].detach().numpy()[rows])
+    np.testing.assert_array_equal(got["emb.weights.1"], m.emb.weights[1].detach().numpy())
+    assert len(got["plain.weights.0.rows"]) == bench.DUMP_ROWS
+    for f in os.listdir(tmp_path / "a"):
+        np.testing.assert_array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f))
+
+
 def _profile_lines():
     import glob
     for path in sorted(glob.glob(os.path.join(ROOT, "profiles", "r2_bench_*.json"))):

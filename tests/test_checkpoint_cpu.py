@@ -2,12 +2,21 @@
 import os
 
 import numpy as np
+import pytest
 import torch
 
 import recommend_tf2_b200 as pkg
 from recommend_tf2_b200 import checkpoint as ck
+from recommend_tf2_b200 import core
 from recommend_tf2_b200.core import DNN, Dense, Layer
 from recommend_tf2_b200.embedding import EmbeddingTables
+
+
+@pytest.fixture(autouse=True)
+def _layers_on_cpu(monkeypatch):
+    """Layers create their weights on CUDA when a device is present; the model here runs on CPU
+    tensors, so it is built on the CPU on every machine."""
+    monkeypatch.setattr(core, "_default_device", lambda: torch.device("cpu"))
 
 
 class TinyDLRM(Layer):
