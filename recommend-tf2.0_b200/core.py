@@ -9,7 +9,6 @@ glorot_uniform kernels, zero biases.
 from __future__ import annotations
 
 import math
-import os
 from typing import Callable, Optional, Sequence
 
 import torch
@@ -155,7 +154,7 @@ class Dense(Layer):
 # the 6 partial products above one fp32 ulp accumulated in fp32; csrc/dense_gemm.cuh), "library" =
 # the framework's GEMM (cuBLAS).  Shapes the tensor-core path does not take (K or N not a multiple
 # of 4, tiny problems, CPU tensors) always use the library.
-DENSE_GEMM = os.environ.get("RTF_DENSE_GEMM", "bf16x6")
+DENSE_GEMM = "bf16x6"
 
 
 def set_dense_gemm(kind: str) -> None:

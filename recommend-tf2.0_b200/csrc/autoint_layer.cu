@@ -24,8 +24,6 @@
 //                                   CTA's samples (fixed grid, fixed order); the per-CTA
 //                                   partials are summed in CTA order by a second tiny kernel,
 // so the weight gradients are reproducible bit for bit.
-#include <cstdlib>
-
 #include "rtf_common.cuh"
 
 namespace rtf {
@@ -168,73 +166,16 @@ __device__ __forceinline__ void ai_load_x(const float* __restrict__ src, float* 
     *reinterpret_cast<float4*>(Xs + e) = ldg_nc_f4(src + e);
 }
 
-template <int DM, int HS, int HSZ>
-__global__ void __launch_bounds__(AI_THREADS, 4)
-autoint_fwd_kernel(const __grid_constant__ AiParams P) {
-  extern __shared__ __align__(16) float sm[];
-  const int F = P.F, H = P.H;
-  const int kMat = F * HS, kS = F | 1;
-  float* Xs = sm;                        // [F][DM]
-  float* Ms = Xs + F * DM;               // Q | K | V | R, each [F][HS]
-  float* Ps = Ms + 4 * kMat;             // [H][F][kS]
-  const int lane = threadIdx.x & 31, m = threadIdx.x >> 5;
-  const bool live = m < 3 || P.use_res;
-  float wreg[(HS + 31) / 32][DM];
-  ai_load_weights<DM, HS>(P, wreg, m, lane, live);
-  for (long long b = blockIdx.x; b < P.B; b += gridDim.x) {
-    ai_load_x<DM, HS>(P.x + b * F * DM, Xs, F * DM);
-    __syncthreads();
-    ai_project<DM, HS>(Xs, Ms, wreg, F, P.act, m, lane, live);
-    __syncthreads();
-    for (int p = threadIdx.x; p < H * F; p += AI_THREADS) {
-      const int h = p / F, i = p - h * F;
-      ai_scores<DM, HS, HSZ>(Ms, Ps, F, h, i, P.scale);
-      const float* prow = Ps + (h * F + i) * kS;
-      const float* V = Ms + 2 * kMat + h * HSZ;
-      float o[HSZ];
-#pragma unroll
-      for (int d = 0; d < HSZ; ++d) o[d] = 0.f;
-      for (int j = 0; j < F; ++j) {
-        const float pj = prow[j];
-        const float4* vr = reinterpret_cast<const float4*>(V + j * HS);
-#pragma unroll
-        for (int d4 = 0; d4 < HSZ / 4; ++d4) {
-          const float4 vv = vr[d4];
-          o[4 * d4] = fmaf(pj, vv.x, o[4 * d4]);
-          o[4 * d4 + 1] = fmaf(pj, vv.y, o[4 * d4 + 1]);
-          o[4 * d4 + 2] = fmaf(pj, vv.z, o[4 * d4 + 2]);
-          o[4 * d4 + 3] = fmaf(pj, vv.w, o[4 * d4 + 3]);
-        }
-      }
-      float* dst = P.out + (b * F + i) * HS + h * HSZ;
-      const float* R = Ms + 3 * kMat + i * HS + h * HSZ;
-#pragma unroll
-      for (int d4 = 0; d4 < HSZ / 4; ++d4) {
-        float4 v = make_float4(o[4 * d4], o[4 * d4 + 1], o[4 * d4 + 2], o[4 * d4 + 3]);
-        if (P.use_res) {
-          const float4 r = *reinterpret_cast<const float4*>(R + 4 * d4);
-          v.x = fmaxf(v.x + r.x, 0.f);
-          v.y = fmaxf(v.y + r.y, 0.f);
-          v.z = fmaxf(v.z + r.z, 0.f);
-          v.w = fmaxf(v.w + r.w, 0.f);
-        }
-        *reinterpret_cast<float4*>(dst + 4 * d4) = v;
-      }
-    }
-    __syncthreads();  // Xs / Ms / Ps are overwritten by the next sample
-  }
-}
-
-// ---- forward, packed-FMA version (sm_100 FFMA2: two fp32 FMAs per issue slot) ----------------
-// The scalar version above is bound by the FMA pipe's issue rate (one FFMA per 2 cycles and
-// scheduler).  Here every contraction is arranged so that BOTH halves of a packed FMA are useful
-// and come out of the loads already paired:
+// ---- forward, packed FMAs (sm_100 FFMA2: two fp32 FMAs per issue slot) -----------------------
+// Scalar FFMA, as in ai_project / ai_scores above, is bound by the FMA pipe's issue rate (one FFMA
+// per 2 cycles and scheduler).  Here every contraction is arranged so that BOTH halves of a packed
+// FMA are useful and come out of the loads already paired:
 //   projections: X is staged TRANSPOSED (Xt[k][row]), one 128-bit broadcast load gives 4 rows of
 //                column k = two row pairs; {w,w} pairs live in registers for the whole launch;
 //   Q K^T:       K is written transposed by its projection (Kt[col][key]); a thread owns a query
 //                row, keeps its scores in REGISTERS (FP/2 float2) and adds {q_d,q_d} x {K_j,K_j+1};
 //   P V:         pairs over the head dimension come straight from V's rows, {p,p} is one move.
-// FP = compile-time bound on the field count (multiple of 4); softmax as in the scalar version.
+// FP = compile-time bound on the field count (multiple of 4); softmax as in ai_scores.
 template <int DM, int HS, int HSZ, int FP>
 __global__ void __launch_bounds__(AI_THREADS, FP <= 40 ? 4 : 2)
 autoint_fwd2_kernel(const __grid_constant__ AiParams P) {
@@ -590,10 +531,6 @@ autoint_dw_reduce(const float* __restrict__ partial, int ncta, int n, float* __r
 
 static size_t ai_round16(size_t nfloats) { return (nfloats + 3) / 4 * 4 * sizeof(float); }
 template <int DM, int HS>
-static size_t ai_fwd_smem(int F, int H) {
-  return ai_round16((size_t)F * DM + 4 * (size_t)F * HS + (size_t)H * F * (F | 1));
-}
-template <int DM, int HS>
 static size_t ai_bwd_smem(int F, int H) {
   return ai_round16((size_t)F * DM + 5 * (size_t)F * HS + 2 * (size_t)H * F * (F | 1));
 }
@@ -621,23 +558,9 @@ static int ai_launch_fwd2(const AiParams& P, cudaStream_t st) {
 
 template <int DM, int HS, int HSZ>
 static int ai_launch_fwd(const AiParams& P, cudaStream_t st) {
-  static const bool scalar = getenv("RTF_K6_SCALAR") != nullptr;   // comparison runs only
-  if (!scalar) {
-    if (P.F <= 16) return ai_launch_fwd2<DM, HS, HSZ, 16>(P, st);
-    if (P.F <= 40) return ai_launch_fwd2<DM, HS, HSZ, 40>(P, st);
-    return ai_launch_fwd2<DM, HS, HSZ, 64>(P, st);
-  }
-  const size_t smem = ai_fwd_smem<DM, HS>(P.F, P.H);
-  if (smem > 227 * 1024) return RTF_E_RANGE;
-  cudaError_t e = cudaFuncSetAttribute(autoint_fwd_kernel<DM, HS, HSZ>,
-                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  int per_sm = (int)((227 * 1024) / (smem + 1024));
-  if (per_sm > 6) per_sm = 6;
-  if (per_sm < 1) per_sm = 1;
-  autoint_fwd_kernel<DM, HS, HSZ><<<ai_grid(P.B, per_sm), AI_THREADS, smem, st>>>(P);
-  RTF_CHECK_LAUNCH();
-  return 0;
+  if (P.F <= 16) return ai_launch_fwd2<DM, HS, HSZ, 16>(P, st);
+  if (P.F <= 40) return ai_launch_fwd2<DM, HS, HSZ, 40>(P, st);
+  return ai_launch_fwd2<DM, HS, HSZ, 64>(P, st);
 }
 
 }  // namespace rtf

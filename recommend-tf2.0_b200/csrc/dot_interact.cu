@@ -13,7 +13,6 @@
 // a warp hit distinct banks.  Backward re-gathers X (cheaper than saving it) and forms
 // dX = (S + S^T) X with lanes owning 4 embedding columns each.
 // Bound: HBM (ids + rows in, D+P floats out) with the fp32 FMA pipe close behind (DESIGN.md).
-#include <cstdlib>
 #include <type_traits>
 
 #include "rtf_common.cuh"
@@ -51,8 +50,6 @@ struct DotParams {
   long long sample0;           // bwd: global index of this rank's first sample
   int peer_G;
   int32_t* err;
-  int dbg;  // 0 in the product build.  With -DRTF_DOT_EXPERIMENTS, RTF_DOT_DBG sets bits that switch
-            // phases off to time the others: 1 = FMA loop, 2 = row gather, 4 = bwd S fill
 };
 
 __device__ __forceinline__ void peer_split(const DotParams& P, int f, long long id, int& g,
@@ -176,13 +173,13 @@ dot_fwd_kernel(const __grid_constant__ DotParams P, int warp_floats) {
   const long long stride = (long long)gridDim.x * nwarps;
   long long b = (long long)blockIdx.x * nwarps + warp;
   uint32_t parity = 0;
-  if (b < P.B && !(P.dbg & 2)) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
+  if (b < P.B) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
   const int nblk = nbr * (nbr + 1) / 2;
 
   for (; b < P.B; b += stride) {
-    if (!(P.dbg & 2)) mbar_wait(bar, parity);
+    mbar_wait(bar, parity);
     parity ^= 1;
-    for (int blk = lane; blk < ((P.dbg & 1) ? 0 : nblk); blk += 32) {
+    for (int blk = lane; blk < nblk; blk += 32) {
       int bi, bj;
       tri_block(blk, bi, bj);
       // block (bi,bj) covers rows {bi + r*nbr} x {bj + c*nbr}
@@ -237,7 +234,7 @@ dot_fwd_kernel(const __grid_constant__ DotParams P, int warp_floats) {
       }
     }
     __syncwarp();  // every lane is done reading xt/zst before the next sample overwrites them
-    if (b + stride < P.B && !(P.dbg & 2)) dot_issue_rows<IdT>(P, b + stride, xt, RS, bar, lane);
+    if (b + stride < P.B) dot_issue_rows<IdT>(P, b + stride, xt, RS, bar, lane);
   }
 }
 
@@ -298,7 +295,7 @@ dot_fwd7_kernel(const __grid_constant__ DotParams P, int warp_floats) {
   const long long stride = (long long)gridDim.x * nwarps;
   long long b = (long long)blockIdx.x * nwarps + warp;
   uint32_t parity = 0;
-  if (b < P.B && !(P.dbg & 2)) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
+  if (b < P.B) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
   constexpr int rstep = nbr * RS;
   constexpr int nd2 = D >> 1;
   const float* pa = xt + bi * RS;
@@ -306,9 +303,9 @@ dot_fwd7_kernel(const __grid_constant__ DotParams P, int warp_floats) {
   float* zd = Z + bi * ZS + bj;      // Z[i][j]
 
   for (; b < P.B; b += stride) {
-    if (!(P.dbg & 2)) mbar_wait(bar, parity);
+    mbar_wait(bar, parity);
     parity ^= 1;
-    const bool more = b + stride < P.B && !(P.dbg & 2);
+    const bool more = b + stride < P.B;
     const float* src[2] = {nullptr, nullptr};
     if (more) dot_resolve_rows<IdT>(P, b + stride, lane, src);   // id loads fly under the Gram loop
     float2 acc[7][7];
@@ -316,7 +313,7 @@ dot_fwd7_kernel(const __grid_constant__ DotParams P, int warp_floats) {
     for (int r = 0; r < 7; ++r)
 #pragma unroll
       for (int c = 0; c < 7; ++c) acc[r][c] = make_float2(0.f, 0.f);
-    if (grp < ngrp && !(P.dbg & 1)) {
+    if (grp < ngrp) {
 #pragma unroll 1
       for (int e = grp; e < nd2; e += ngrp) {
         float2 a[7], q[7];
@@ -375,136 +372,6 @@ dot_fwd7_kernel(const __grid_constant__ DotParams P, int warp_floats) {
   }
 }
 
-#ifdef RTF_DOT_EXPERIMENTS  // measured-slower variants: records in profiles/, not in the default build
-// Forward, variant 2 (D % 8 == 0; opt-in with RTF_DOT_FWD_V2=1, parity tests pass with it).
-// Measured on B200, DLRM configuration: 0.418 ms vs 0.368 ms for variant 1 — the 25 % fewer
-// shared-memory wavefronts do not pay for the 64-accumulator tile (128 registers + spill, one
-// shuffle per Gram entry, half the independent FFMA2 chains per loaded operand); kept as the
-// record of that experiment.  The 4x4 blocks of one block-row are paired into 4x8 tiles
-// (12 LDS.128 per 64 FFMA2 instead of 8 per 32) and the two half-warps split the embedding
-// dimension, so all 32 lanes stay busy with 16 tiles (27 fields -> 7 block-rows -> 16 tiles) and
-// the shared-memory wavefronts per sample drop from 1024 to 768; the two halves are combined
-// with one shuffle per Gram entry.  Same row interleave (stride nbr) as variant 1, so the
-// 128-bit loads of a quarter-warp still hit distinct banks or broadcast.
-template <typename IdT>
-__global__ void __launch_bounds__(512, 1)
-dot_fwd_kernel_v2(const __grid_constant__ DotParams P, int warp_floats, int cta_floats) {
-  extern __shared__ __align__(16) float smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-  const int F1 = P.F1, D = P.D;
-  const int F1p = (F1 + 3) & ~3, nbr = F1p >> 2;
-  const int RS = dot_row_stride(D);
-  const int npairs = F1 * (F1 - 1) / 2;
-  unsigned char* tile_tab = reinterpret_cast<unsigned char*>(smem);  // [ntiles][2] = (bi, pj)
-  float* xt = smem + cta_floats + (size_t)warp * warp_floats;
-  float* zst = xt + F1p * RS;
-  uint64_t* bar = reinterpret_cast<uint64_t*>(zst + ((npairs + 3) & ~3));
-
-  int ntiles = 0;
-  for (int bi = 0; bi < nbr; ++bi) ntiles += (bi + 2) >> 1;
-  for (int t = threadIdx.x; t < ntiles; t += blockDim.x) {
-    int bi = 0, first = 0;
-    while (first + ((bi + 2) >> 1) <= t) {
-      first += (bi + 2) >> 1;
-      ++bi;
-    }
-    tile_tab[2 * t] = (unsigned char)bi;
-    tile_tab[2 * t + 1] = (unsigned char)(t - first);
-  }
-  if (lane == 0) {
-    mbar_init(bar, 1);
-    mbar_fence_init();
-  }
-  for (int i = F1 * RS + lane; i < F1p * RS; i += 32) xt[i] = 0.f;  // pad rows stay zero
-  __syncthreads();
-
-  const long long stride = (long long)gridDim.x * nwarps;
-  long long b = (long long)blockIdx.x * nwarps + warp;
-  uint32_t parity = 0;
-  if (b < P.B) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
-  const int h = lane >> 4;                      // which half of the embedding dimension
-  const int d0 = h * (D >> 1), d1 = d0 + (D >> 1);
-  const int rstep = nbr * RS;
-
-  for (; b < P.B; b += stride) {
-    mbar_wait(bar, parity);
-    parity ^= 1;
-    for (int t0 = 0; t0 < ntiles; t0 += 16) {   // uniform trip count: every lane shuffles
-      const int tl = t0 + (lane & 15);
-      const bool live = tl < ntiles;
-      const int tc = live ? tl : ntiles - 1;
-      const int bi = tile_tab[2 * tc], bj0 = 2 * tile_tab[2 * tc + 1];
-      const bool has1 = bj0 + 1 <= bi;
-      const int bj1 = has1 ? bj0 + 1 : bj0;
-      float2 acc[4][8];
-#pragma unroll
-      for (int r = 0; r < 4; ++r)
-#pragma unroll
-        for (int c = 0; c < 8; ++c) acc[r][c] = make_float2(0.f, 0.f);
-      const float* pa = xt + bi * RS;
-      const float* pb0 = xt + bj0 * RS;
-      const float* pb1 = xt + bj1 * RS;
-      for (int d = d0; d < d1; d += 4) {
-        float4 a[4], q[4];
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-          a[r] = *reinterpret_cast<const float4*>(pa + r * rstep + d);
-          q[r] = *reinterpret_cast<const float4*>(pb0 + r * rstep + d);
-        }
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            acc[r][c] = __ffma2_rn(make_float2(a[r].x, a[r].y), make_float2(q[c].x, q[c].y), acc[r][c]);
-            acc[r][c] = __ffma2_rn(make_float2(a[r].z, a[r].w), make_float2(q[c].z, q[c].w), acc[r][c]);
-          }
-#pragma unroll
-        for (int r = 0; r < 4; ++r) q[r] = *reinterpret_cast<const float4*>(pb1 + r * rstep + d);
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-#pragma unroll
-          for (int c = 0; c < 4; ++c) {
-            acc[r][4 + c] = __ffma2_rn(make_float2(a[r].x, a[r].y), make_float2(q[c].x, q[c].y), acc[r][4 + c]);
-            acc[r][4 + c] = __ffma2_rn(make_float2(a[r].z, a[r].w), make_float2(q[c].z, q[c].w), acc[r][4 + c]);
-          }
-      }
-      // combine the two halves of d; half 0 then stores block (bi, bj0), half 1 block (bi, bj1)
-#pragma unroll
-      for (int r = 0; r < 4; ++r)
-#pragma unroll
-        for (int c = 0; c < 8; ++c) {
-          float z = acc[r][c].x + acc[r][c].y;
-          z += __shfl_xor_sync(0xffffffffu, z, 16);
-          const bool mine = (c < 4) ? (h == 0) : (h == 1 && has1);
-          if (live && mine) {
-            const int bj = (c < 4) ? bj0 : bj1;
-            const int i = bi + r * nbr, j = bj + (c & 3) * nbr;
-            if (i < F1 && j < i) zst[i * (i - 1) / 2 + j] = z;
-            else if (bi != bj && j < F1 && i < j) zst[j * (j - 1) / 2 + i] = z;
-          }
-        }
-    }
-    __syncwarp();
-    float* o = P.out + b * P.out_sb;
-    for (int d = lane; d < D; d += 32) o[d] = xt[d];
-    for (int p = lane; p < npairs; p += 32) o[D + p] = zst[p];
-    for (int p = D + npairs + lane; p < P.out_cols; p += 32) o[p] = 0.f;
-    if (P.xsave) {
-      float* xs = P.xsave + b * P.xsave_sb;
-      const int nv = D >> 2;
-      for (int e = lane; e < (F1 - 1) * nv; e += 32) {
-        const int r = e / nv, c = e - r * nv;
-        *reinterpret_cast<float4*>(xs + r * D + 4 * c) =
-            *reinterpret_cast<const float4*>(xt + (r + 1) * RS + 4 * c);
-      }
-    }
-    __syncwarp();  // every lane is done reading xt/zst before the next sample overwrites them
-    if (b + stride < P.B) dot_issue_rows<IdT>(P, b + stride, xt, RS, bar, lane);
-  }
-}
-
-#endif  // RTF_DOT_EXPERIMENTS
-
 // backward: dX[i] = sum_j S[i][j] X[j],  S symmetric from dZ, plus the passthrough on row 0
 // row pairs of the t-th 8-row tile of an F1-row sample (the last tile only the pairs that exist)
 __host__ __device__ constexpr int bwd_tile_rpn(int f1, int t) {
@@ -551,7 +418,7 @@ dot_bwd_kernel(const __grid_constant__ DotParams P, int warp_floats) {
   const long long stride = (long long)gridDim.x * nwarps;
   long long b = (long long)blockIdx.x * nwarps + warp;
   uint32_t parity = 0;
-  if (b < P.B && !(P.dbg & 2)) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
+  if (b < P.B) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
   // the incoming gradient of the NEXT sample is fetched into registers while this one is being
   // processed (its HBM latency was a serial 0.07 ms in front of every sample's S fill)
   constexpr int PF = 12;                     // covers F1 <= 28; longer tails are loaded in place
@@ -577,34 +444,32 @@ dot_bwd_kernel(const __grid_constant__ DotParams P, int warp_floats) {
         long long id = (long long)__ldg((const IdT*)P.ids + b * P.ids_sb + (long long)f * P.ids_sf);
         ids_w[f] = (id < 0 || id >= P.rows[f]) ? -1 : id;
       }
-    if (!(P.dbg & 4)) {
 #pragma unroll
-      for (int q = 0; q < PF; ++q) {
-        const int p = lane + 32 * q;
-        if (p < npairs) {
-          const int ij = pair_ij[p];
-          const int i = ij >> 8, j = ij & 255;
-          S[i * SS + j] = gpre[q];
-          S[j * SS + i] = gpre[q];
-        }
-      }
-      for (int p = lane + 32 * PF; p < npairs; p += 32) {
-        const float v = __ldg(g + D + p);
+    for (int q = 0; q < PF; ++q) {
+      const int p = lane + 32 * q;
+      if (p < npairs) {
         const int ij = pair_ij[p];
         const int i = ij >> 8, j = ij & 255;
-        S[i * SS + j] = v;
-        S[j * SS + i] = v;
+        S[i * SS + j] = gpre[q];
+        S[j * SS + i] = gpre[q];
       }
+    }
+    for (int p = lane + 32 * PF; p < npairs; p += 32) {
+      const float v = __ldg(g + D + p);
+      const int ij = pair_ij[p];
+      const int i = ij >> 8, j = ij & 255;
+      S[i * SS + j] = v;
+      S[j * SS + i] = v;
     }
     const float4 g0 = g0pre;
     const bool more = b + stride < P.B;
     const float* src[2] = {nullptr, nullptr};
     if (more) {
       prefetch(b + stride);
-      if (!(P.dbg & 2)) dot_resolve_rows<IdT>(P, b + stride, lane, src);  // id loads fly under the FMA loop
+      dot_resolve_rows<IdT>(P, b + stride, lane, src);  // id loads fly under the FMA loop
     }
     __syncwarp();
-    if (!(P.dbg & 2)) mbar_wait(bar, parity);
+    mbar_wait(bar, parity);
     parity ^= 1;
     // one i-tile of 2*RPN rows (RPN = 4 except for the last tile, which only computes the row
     // pairs that exist: 27 rows = 8 + 8 + 8 + 4, not 32).
@@ -620,7 +485,7 @@ dot_bwd_kernel(const __grid_constant__ DotParams P, int warp_floats) {
 #pragma unroll
         for (int c = 0; c < 4; ++c) acc2[rp][c] = make_float2(0.f, 0.f);
 #pragma unroll (CF1 ? CF1 : 3)
-      for (int j = 0; j < ((P.dbg & 1) ? 0 : F1); ++j) {
+      for (int j = 0; j < F1; ++j) {
         const float4 xj = *reinterpret_cast<const float4*>(xt + j * RS + d0);
         const float4 s0 = *reinterpret_cast<const float4*>(S + j * SS + i0);
         float4 s1 = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -685,245 +550,9 @@ dot_bwd_kernel(const __grid_constant__ DotParams P, int warp_floats) {
       }
     }
     __syncwarp();
-    if (more && !(P.dbg & 2)) dot_issue_resolved(P, xt, RS, bar, lane, src);
+    if (more) dot_issue_resolved(P, xt, RS, bar, lane, src);
   }
 }
-
-#ifdef RTF_DOT_EXPERIMENTS
-// ------------------------------------------------------------------------------------------
-// Tensor-core variants for F1 <= 32, D % 8 == 0 (the DLRM shape: 27 x 128).
-//
-// The FFMA kernels above are bound by instruction issue (ncu: issue slots 59 %, FMA pipe 37 %,
-// DRAM 15 %: 3 458 warp instructions per sample for 1 404 useful FFMA).  A single-pass TF32 MMA
-// would break the 1e-5 fp32 parity bar, so each operand is split x = hi + lo (two TF32 values,
-// ~22 mantissa bits) and every product is three m16n8k8 MMAs (hi*hi + hi*lo + lo*hi, fp32
-// accumulate) — "3xTF32", error ~2^-21 of |x_i||x_j|.  The per-sample Gram (M = N = 32) is far
-// below tcgen05's M >= 64 tile, so this is warp-level mma.sync (one warp still owns one sample,
-// rows still arrive by TMA bulk copies); ~4x fewer issue slots than the FFMA form.
-// Fragment trick: for Z = X X^T the B fragment of an 8-row n-tile is a relabelling of the A
-// fragment registers of the 16-row m-tile that contains it, so X is read from shared memory once.
-__device__ __forceinline__ uint32_t f2tf32(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return r;
-}
-__device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
-  hi = f2tf32(x);
-  lo = f2tf32(x - __uint_as_float(hi));
-}
-__device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], uint32_t b0,
-                                         uint32_t b1) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, "
-      "{%0,%1,%2,%3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
-}
-// c += A*B with A, B given as hi/lo pairs (small terms first)
-__device__ __forceinline__ void mma3(float (&c)[4], const uint32_t (&ah)[4], const uint32_t (&al)[4],
-                                     uint32_t bh0, uint32_t bh1, uint32_t bl0, uint32_t bl1) {
-  mma_tf32(c, al, bh0, bh1);
-  mma_tf32(c, ah, bl0, bl1);
-  mma_tf32(c, ah, bh0, bh1);
-}
-
-__host__ __device__ inline int dot_row_stride_bwd(int D) { return D + ((D % 32 == 24) ? 16 : 8); }
-
-template <typename IdT>
-__global__ void __launch_bounds__(512, 1)
-dot_fwd_mma_kernel(const __grid_constant__ DotParams P, int warp_floats) {
-  extern __shared__ __align__(16) float smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-  const int g = lane >> 2, t = lane & 3;
-  const int F1 = P.F1, D = P.D;
-  const int RS = dot_row_stride(D);
-  const int npairs = F1 * (F1 - 1) / 2;
-  float* xt = smem + (size_t)warp * warp_floats;  // [32][RS], rows >= F1 stay zero
-  float* zst = xt + 32 * RS;
-  uint64_t* bar = reinterpret_cast<uint64_t*>(zst + ((npairs + 3) & ~3));
-  if (lane == 0) {
-    mbar_init(bar, 1);
-    mbar_fence_init();
-  }
-  for (int i = F1 * RS + lane; i < 32 * RS; i += 32) xt[i] = 0.f;
-  __syncwarp();
-  const long long stride = (long long)gridDim.x * nwarps;
-  long long b = (long long)blockIdx.x * nwarps + warp;
-  uint32_t parity = 0;
-  if (b < P.B) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
-  const bool two_mt = F1 > 16;
-
-  for (; b < P.B; b += stride) {
-    mbar_wait(bar, parity);
-    parity ^= 1;
-    // tiles (m-tile, n-tile): (0,0) (0,1) (1,0) (1,1) (1,2) (1,3)
-    float acc[6][4];
-#pragma unroll
-    for (int i = 0; i < 6; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-    const float* r0 = xt + g * RS + t;
-#pragma unroll 2
-    for (int k0 = 0; k0 < D; k0 += 8) {
-      uint32_t ah[2][4], al[2][4];
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt) {
-        if (mt == 1 && !two_mt) {
-#pragma unroll
-          for (int q = 0; q < 4; ++q) ah[1][q] = al[1][q] = 0u;
-          continue;
-        }
-        const float* p = r0 + mt * 16 * RS + k0;
-        split_tf32(p[0], ah[mt][0], al[mt][0]);
-        split_tf32(p[8 * RS], ah[mt][1], al[mt][1]);
-        split_tf32(p[4], ah[mt][2], al[mt][2]);
-        split_tf32(p[8 * RS + 4], ah[mt][3], al[mt][3]);
-      }
-      // n-tile nt of 8 rows: nt = 2*mt' + h  ->  B regs = A regs (h, h+2) of m-tile mt'
-      mma3(acc[0], ah[0], al[0], ah[0][0], ah[0][2], al[0][0], al[0][2]);
-      mma3(acc[1], ah[0], al[0], ah[0][1], ah[0][3], al[0][1], al[0][3]);
-      if (two_mt) {
-        mma3(acc[2], ah[1], al[1], ah[0][0], ah[0][2], al[0][0], al[0][2]);
-        mma3(acc[3], ah[1], al[1], ah[0][1], ah[0][3], al[0][1], al[0][3]);
-        mma3(acc[4], ah[1], al[1], ah[1][0], ah[1][2], al[1][0], al[1][2]);
-        mma3(acc[5], ah[1], al[1], ah[1][1], ah[1][3], al[1][1], al[1][3]);
-      }
-    }
-    // scatter the lower triangle into the staging row: c0 (g,2t) c1 (g,2t+1) c2 (g+8,2t) c3 (g+8,2t+1)
-#pragma unroll
-    for (int tile = 0; tile < 6; ++tile) {
-      const int mt = tile < 2 ? 0 : 1, nt = tile < 2 ? tile : tile - 2;
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        const int i = mt * 16 + g + ((q & 2) ? 8 : 0);
-        const int j = nt * 8 + 2 * t + (q & 1);
-        if (i < F1 && j < i) zst[i * (i - 1) / 2 + j] = acc[tile][q];
-      }
-    }
-    __syncwarp();
-    float* o = P.out + b * P.out_sb;
-    for (int d = lane; d < D; d += 32) o[d] = xt[d];
-    for (int p = lane; p < npairs; p += 32) o[D + p] = zst[p];
-    for (int p = D + npairs + lane; p < P.out_cols; p += 32) o[p] = 0.f;
-    __syncwarp();
-    if (b + stride < P.B) dot_issue_rows<IdT>(P, b + stride, xt, RS, bar, lane);
-  }
-}
-
-template <typename IdT>
-__global__ void __launch_bounds__(512, 1)
-dot_bwd_mma_kernel(const __grid_constant__ DotParams P, int warp_floats) {
-  extern __shared__ __align__(16) float smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
-  const int g = lane >> 2, t = lane & 3;
-  const int F1 = P.F1, D = P.D;
-  const int RS = dot_row_stride_bwd(D);
-  constexpr int SS = 36;  // S row stride: 4g + t hits 32 distinct banks
-  const int npairs = F1 * (F1 - 1) / 2;
-  unsigned short* pair_ij = reinterpret_cast<unsigned short*>(smem);
-  const int pair_floats = ((npairs + 1) / 2 + 3) & ~3;
-  float* xt = smem + pair_floats + (size_t)warp * warp_floats;  // [32][RS]
-  float* S = xt + 32 * RS;                                      // [32][SS]
-  uint64_t* bar = reinterpret_cast<uint64_t*>(S + 32 * SS);
-  for (int p = threadIdx.x; p < npairs; p += blockDim.x) {
-    int i = (int)((1.f + sqrtf(1.f + 8.f * p)) * 0.5f);
-    while (i * (i - 1) / 2 > p) --i;
-    while ((i + 1) * i / 2 <= p) ++i;
-    pair_ij[p] = (unsigned short)((i << 8) | (p - i * (i - 1) / 2));
-  }
-  if (lane == 0) {
-    mbar_init(bar, 1);
-    mbar_fence_init();
-  }
-  for (int i = F1 * RS + lane; i < 32 * RS; i += 32) xt[i] = 0.f;
-  for (int i = lane; i < 32 * SS; i += 32) S[i] = 0.f;
-  __syncthreads();
-  const long long stride = (long long)gridDim.x * nwarps;
-  long long b = (long long)blockIdx.x * nwarps + warp;
-  uint32_t parity = 0;
-  if (b < P.B) dot_issue_rows<IdT>(P, b, xt, RS, bar, lane);
-  const int n_mt = F1 > 16 ? 2 : 1;
-  const int n_ks = (F1 + 7) >> 3;
-
-  for (; b < P.B; b += stride) {
-    const float* gr = P.gout + b * P.gout_sb;
-    for (int p = lane; p < npairs; p += 32) {
-      const float v = __ldg(gr + D + p);
-      const int ij = pair_ij[p];
-      const int i = ij >> 8, j = ij & 255;
-      S[i * SS + j] = v;
-      S[j * SS + i] = v;
-    }
-    __syncwarp();
-    // A fragments of S (hi/lo), kept in registers for the whole sample
-    uint32_t sh[2][4][4], sl[2][4][4];
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks) {
-        const float* p = S + (mt * 16 + g) * SS + ks * 8 + t;
-        split_tf32(p[0], sh[mt][ks][0], sl[mt][ks][0]);
-        split_tf32(p[8 * SS], sh[mt][ks][1], sl[mt][ks][1]);
-        split_tf32(p[4], sh[mt][ks][2], sl[mt][ks][2]);
-        split_tf32(p[8 * SS + 4], sh[mt][ks][3], sl[mt][ks][3]);
-      }
-    mbar_wait(bar, parity);
-    parity ^= 1;
-    for (int n0 = 0; n0 < D; n0 += 32) {  // 4 n-tiles of 8 columns per chunk
-      float acc[2][4][4];
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-          for (int q = 0; q < 4; ++q) acc[mt][nt][q] = 0.f;
-#pragma unroll
-      for (int ks = 0; ks < 4; ++ks) {
-        if (ks >= n_ks) break;
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
-          const int n = n0 + nt * 8 + g;
-          uint32_t bh0 = 0, bh1 = 0, bl0 = 0, bl1 = 0;
-          if (n < D) {
-            split_tf32(xt[(ks * 8 + t) * RS + n], bh0, bl0);
-            split_tf32(xt[(ks * 8 + t + 4) * RS + n], bh1, bl1);
-          }
-          mma3(acc[0][nt], sh[0][ks], sl[0][ks], bh0, bh1, bl0, bl1);
-          if (n_mt > 1) mma3(acc[1][nt], sh[1][ks], sl[1][ks], bh0, bh1, bl0, bl1);
-        }
-      }
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-          for (int h = 0; h < 2; ++h) {
-            const int i = mt * 16 + g + h * 8;
-            const int c = n0 + nt * 8 + 2 * t;
-            if (i < F1 && c < D) {
-              float2 v = make_float2(acc[mt][nt][2 * h], acc[mt][nt][2 * h + 1]);
-              if (i == 0) {  // out[:, :D] is X[0] itself
-                v.x += __ldg(gr + c);
-                v.y += __ldg(gr + c + 1);
-              }
-              *reinterpret_cast<float2*>(P.gbase[i] + b * P.gstride[i] + c) = v;
-            }
-          }
-    }
-    __syncwarp();
-    if (b + stride < P.B) dot_issue_rows<IdT>(P, b + stride, xt, RS, bar, lane);
-  }
-}
-
-static bool dot_use_mma(int F1, int D) {
-  // measured on B200 (profiles/README.md): legacy mma.sync TF32 runs at ~20 cycles per m16n8k8
-  // per SM sub-partition, so 3xTF32 is no faster than packed FFMA2 forward (0.35 vs 0.38 ms)
-  // and 2x slower backward; opt-in for experiments only.
-  static const bool use_mma = getenv("RTF_DOT_MMA") != nullptr;
-  return use_mma && F1 <= 32 && D % 8 == 0;
-}
-
-#endif  // RTF_DOT_EXPERIMENTS
 
 static int dot_check_common(long long B, int F1, int D) {
   if (B < 0 || F1 < 2 || D <= 0) return RTF_E_ARG;
@@ -949,88 +578,28 @@ static int dot_launch(Kern kern, const DotParams& P, int warp_floats, int cta_fl
   return 0;
 }
 
-#ifdef RTF_DOT_EXPERIMENTS
-template <typename Kern>
-static int dot_launch_v2(Kern kern, const DotParams& P, int warp_floats, int cta_floats,
-                         cudaStream_t st) {
-  const size_t max_smem = 227 * 1024;
-  const size_t per_warp = (size_t)warp_floats * 4;
-  int nwarps = (int)((max_smem - (size_t)cta_floats * 4) / per_warp);
-  if (nwarps < 1) return RTF_E_RANGE;
-  if (nwarps > 16) nwarps = 16;
-  const size_t smem = (size_t)cta_floats * 4 + per_warp * nwarps;
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  long long blocks = (P.B + nwarps - 1) / nwarps;
-  if (blocks > kNumSMs) blocks = kNumSMs;  // persistent: one CTA per SM
-  kern<<<(unsigned)blocks, nwarps * 32, smem, st>>>(P, warp_floats, cta_floats);
-  RTF_CHECK_LAUNCH();
-  return 0;
-}
-
-static bool dot_use_fwd_v2(int D) {
-  // off by default: measured slower than variant 1 (see the kernel's header comment)
-  static const bool on = getenv("RTF_DOT_FWD_V2") != nullptr;
-  return on && D % 8 == 0;
-}
-
-#endif  // RTF_DOT_EXPERIMENTS
-
 static int dot_fwd_impl(DotParams& P, int ids_i64, cudaStream_t st) {
-#ifdef RTF_DOT_EXPERIMENTS   // phase-isolation switches (wrong results by design): experiments only
-  static const int dbg = getenv("RTF_DOT_DBG") ? atoi(getenv("RTF_DOT_DBG")) : 0;
-  P.dbg = dbg;
-#endif
   const int F1p = (P.F1 + 3) & ~3, RS = dot_row_stride(P.D);
   const int npairs = P.F1 * (P.F1 - 1) / 2;
-#ifdef RTF_DOT_EXPERIMENTS
-  if (dot_use_fwd_v2(P.D)) {
-    const int wf = F1p * RS + ((npairs + 3) & ~3) + 4;
-    const int cf = 64;  // tile table: <= 72 tiles x 2 bytes, padded to 256 B
-    return ids_i64 ? dot_launch_v2(dot_fwd_kernel_v2<int64_t>, P, wf, cf, st)
-                   : dot_launch_v2(dot_fwd_kernel_v2<int32_t>, P, wf, cf, st);
-  }
-  if (dot_use_mma(P.F1, P.D) && !P.xsave) {
-    const int wf = 32 * RS + ((npairs + 3) & ~3) + 4;
-    return ids_i64 ? dot_launch(dot_fwd_mma_kernel<int64_t>, P, wf, 0, st)
-                   : dot_launch(dot_fwd_mma_kernel<int32_t>, P, wf, 0, st);
-  }
-#endif
-  {   // 7x7 register blocks (instantiated for the shape the bench and the reference's Criteo
-      // DLRM use; every other shape takes the generic 4x4 kernel)
-    const int nbr7 = (P.F1 + 6) / 7;
-    static const int variant = getenv("RTF_DOT_FWD") ? atoi(getenv("RTF_DOT_FWD")) : 7;
-    if (variant == 7 && nbr7 == 4 && P.D == 128) {     // the Criteo shape: 22..28 rows of 128
-      const int wf = 28 * RS + ((28 * 29 + 3) & ~3) + 4;    // rows, Z tile, mbarrier
-      const int cf = ((npairs + 1) / 2 + 3) & ~3;           // pair table
-      // 12 warps (154 registers each); measured 12 / 11 / 10 / 8 warps: 0.305 / 0.327 / 0.374 / 0.396 ms
-      return ids_i64 ? dot_launch(dot_fwd7_kernel<int64_t, 128, 4>, P, wf, cf, st, 12)
-                     : dot_launch(dot_fwd7_kernel<int32_t, 128, 4>, P, wf, cf, st, 12);
-    }
+  // 7x7 register blocks (instantiated for the shape the bench and the reference's Criteo DLRM
+  // use; every other shape takes the generic 4x4 kernel)
+  if ((P.F1 + 6) / 7 == 4 && P.D == 128) {     // the Criteo shape: 22..28 rows of 128
+    const int wf = 28 * RS + ((28 * 29 + 3) & ~3) + 4;    // rows, Z tile, mbarrier
+    const int cf = ((npairs + 1) / 2 + 3) & ~3;           // pair table
+    // 12 warps (154 registers each); measured 12 / 11 / 10 / 8 warps: 0.305 / 0.327 / 0.374 / 0.396 ms
+    return ids_i64 ? dot_launch(dot_fwd7_kernel<int64_t, 128, 4>, P, wf, cf, st, 12)
+                   : dot_launch(dot_fwd7_kernel<int32_t, 128, 4>, P, wf, cf, st, 12);
   }
   const int warp_floats = F1p * RS + ((npairs + 3) & ~3) + 4;  // + mbarrier (8 B, 16-B slot)
   return ids_i64 ? dot_launch(dot_fwd_kernel<int64_t>, P, warp_floats, 0, st)
                  : dot_launch(dot_fwd_kernel<int32_t>, P, warp_floats, 0, st);
 }
 static int dot_bwd_impl(DotParams& P, int ids_i64, cudaStream_t st) {
-#ifdef RTF_DOT_EXPERIMENTS
-  static const int dbg = getenv("RTF_DOT_DBG") ? atoi(getenv("RTF_DOT_DBG")) : 0;
-  P.dbg = dbg;
-#endif
   const int F1p = (P.F1 + 7) & ~7, RS = dot_row_stride(P.D);
   const int npairs = P.F1 * (P.F1 - 1) / 2;
-#ifdef RTF_DOT_EXPERIMENTS
-  if (dot_use_mma(P.F1, P.D) && !P.peer_gptr) {
-    const int wf = 32 * dot_row_stride_bwd(P.D) + 32 * 36 + 4;
-    const int cf = ((npairs + 1) / 2 + 3) & ~3;
-    return ids_i64 ? dot_launch(dot_bwd_mma_kernel<int64_t>, P, wf, cf, st)
-                   : dot_launch(dot_bwd_mma_kernel<int32_t>, P, wf, cf, st);
-  }
-#endif
   const int warp_floats = P.F1 * RS + P.F1 * (F1p + 4) + 4 + 128;  // + mbarrier slot + 64 ids
   const int cta_floats = ((npairs + 1) / 2 + 3) & ~3;
-  static const int variant = getenv("RTF_DOT_BWD") ? atoi(getenv("RTF_DOT_BWD")) : 1;
-  if (variant == 1 && P.F1 == 27 && P.D == 128)    // the Criteo shape (26 tables + the dense row)
+  if (P.F1 == 27 && P.D == 128)    // the Criteo shape (26 tables + the dense row)
     return ids_i64 ? dot_launch(dot_bwd_kernel<int64_t, 27, 128>, P, warp_floats, cta_floats, st, 12)
                    : dot_launch(dot_bwd_kernel<int32_t, 27, 128>, P, warp_floats, cta_floats, st, 12);
   return ids_i64 ? dot_launch(dot_bwd_kernel<int64_t>, P, warp_floats, cta_floats, st)
