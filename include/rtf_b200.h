@@ -350,6 +350,22 @@ int rtf_bce_workspace(int64_t n, size_t* bytes);
 int rtf_bce_fwd(const float* d_y, const float* d_p, int64_t n, float* d_loss, float* d_dp,
                 void* d_ws, void* stream);
 
+/* ---- Keras AUC() (ROC, interpolation, T evenly spaced thresholds; SURVEY App. A19) -----------
+ * replaces: model.compile(..., metrics=[AUC()]) + model.evaluate — src/ctr/fm/train.py:50,58,67.
+ * bucket(p) = max(ceilf(__fmul_rn(p, T-1)) - 1, 0); d_counts is [2][T] uint64: row 0 positives,
+ * row 1 negatives PER BUCKET (not cumulative).  _update ADDS a batch of n predictions d_pred and
+ * labels d_label (both fp32) to it; the caller zeroes d_counts and *d_err on reset.  An element
+ * with p outside [0,1], p NaN or a label other than 0 / 1 is not counted and sets bit 0 of *d_err.
+ * Shared-memory histogram per CTA, flushed with 64-bit integer atomics: the counts are exact and
+ * independent of the launch order.  n == 0 launches nothing.  2 <= T <= 4096, else RTF_E_RANGE.
+ * _result: tp / fp = integer suffix sums of the buckets, tpr = tp/P, fpr = fp/N (0 when P or N is
+ * 0), AUC = sum_{i<T-1} (fpr[i]-fpr[i+1]) (tpr[i]+tpr[i+1]) / 2 in fp64 in a fixed order, written
+ * as fp32 to *d_auc (device memory: no host sync, capturable in a CUDA graph).                  */
+int rtf_auc_update(const float* d_pred, const float* d_label, int64_t n, int num_thresholds,
+                   unsigned long long* d_counts, int* d_err, void* stream);
+int rtf_auc_result(const unsigned long long* d_counts, int num_thresholds, float* d_auc,
+                   void* stream);
+
 /* ---- BatchNormalization of the DNN block (MLP either side of the path, SURVEY §8 f2) -------
  * replaces: tensorflow.keras.layers.BatchNormalization in training mode at the head of
  *           ctr.layers.modules.DNN (src/ctr/layers/modules.py:129-135; Keras defaults App. A9)

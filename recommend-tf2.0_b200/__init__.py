@@ -15,11 +15,12 @@ from . import models
 from . import data
 from . import retrieval
 from . import checkpoint
+from . import metrics
 from .checkpoint import load_weights, save_weights
 from .retrieval import IndexFlatIP, topk_ip
 from .data import DeviceFeeder, criteo_feature_columns, denseFeature, sparseFeature, varLenSparseFeat
 
 __all__ = ["RtfError", "build", "lib", "EmbeddingTables", "SparseOptimizer", "embed_fwd",
            "embed_bwd", "dot_interact", "dot_out_cols", "embed_dot", "attention", "FM", "FMModel",
-           "colsum", "layers", "retrieval", "IndexFlatIP", "topk_ip", "checkpoint", "save_weights", "load_weights", "DLRM", "DLRMTrainer", "models", "data", "DeviceFeeder",
+           "colsum", "layers", "retrieval", "IndexFlatIP", "topk_ip", "checkpoint", "save_weights", "load_weights", "metrics", "DLRM", "DLRMTrainer", "models", "data", "DeviceFeeder",
            "criteo_feature_columns", "denseFeature", "sparseFeature", "varLenSparseFeat"]

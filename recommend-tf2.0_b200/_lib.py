@@ -71,6 +71,8 @@ SIGNATURES = {
     "rtf_layernorm_bwd": [_p, _p, _p, _p, _p, _i64, _int, _p, _p, _p, _p, C.c_size_t, _p],
     "rtf_bce_workspace": [_i64, C.POINTER(C.c_size_t)],
     "rtf_bce_fwd": [_p, _p, _i64, _p, _p, _p, _p],
+    "rtf_auc_update": [_p, _p, _i64, _int, _p, _p, _p],
+    "rtf_auc_result": [_p, _int, _p, _p],
     "rtf_relu_bwd_colsum_workspace": [_i64, _int, C.POINTER(C.c_size_t)],
     "rtf_relu_bwd_colsum": [_p, _p, _i64, _int, _p, _p, _p, _p],
     "rtf_autoint_layer_supported": [_int, _int, _int, _int],

@@ -76,8 +76,11 @@ class DLRMTrainer:
     optimizer on the tables), dense Adam on the MLPs (Keras form, core.DenseAdam: one
     rtf_dense_adam launch over the flat parameter buffer)."""
 
-    def __init__(self, model: DLRM, lr: float = 1e-3, cuda_graph: bool = False):
+    def __init__(self, model: DLRM, lr: float = 1e-3, cuda_graph: bool = False, metrics=None):
         self.model = model
+        self.metrics = list(metrics or [])      # updated by every step (metrics.AUC)
+        self.cuda_graph = cuda_graph
+        self._evaluator = None
         if model.embed_layers.optimizer is None:
             model.embed_layers.set_optimizer(SparseOptimizer("adam", lr=lr, l2=model.embed_reg))
         self.dense_opt = None
@@ -95,13 +98,15 @@ class DLRMTrainer:
         m = self.model
         pred = m(inputs)
         loss = binary_crossentropy(labels, pred)
+        for mt in self.metrics:
+            mt.update_state(labels, pred.detach())
         self.dense_opt.zero_grad()
         loss.backward()
         self.dense_opt.apply()
         m.embed_layers.wait_pending()   # K2's row update ran on the side stream behind the MLP backward
         return loss.detach()
 
-    def step(self, dense, sparse, labels) -> torch.Tensor:
+    def _setup(self, dense):
         m = self.model
         if self.dense_opt is None:      # layers build on first call: build them, then flatten
             build_dense_layers(m, dense.shape[1], dense.device)
@@ -109,7 +114,25 @@ class DLRMTrainer:
             if self.graph is not None:
                 self.dense_opt.enable_device_lr()
                 m.embed_layers.optimizer.enable_device_lr(dense.device)
+
+    def step(self, dense, sparse, labels) -> torch.Tensor:
+        self._setup(dense)
         if self.graph is not None:
             return self.graph([dense, sparse], labels)
         self._advance()
         return self._body([dense, sparse], labels)
+
+    def _eval_forward(self, inputs, labels):
+        pred = self.model(inputs)
+        return pred, binary_crossentropy(labels, pred)
+
+    def evaluate(self, batches) -> dict:
+        """Keras `model.evaluate` over `(dense, sparse, labels)` batches (as DeviceFeeder yields
+        them): {"loss": batch-size-weighted mean BCE, <metric name>: value, ...}, computed by
+        fresh copies of the trainer's metrics.  Changes no parameter, buffer, table, optimizer
+        state or step counter (metrics.Evaluator)."""
+        if self._evaluator is None:
+            from .metrics import Evaluator
+            self._evaluator = Evaluator(self._eval_forward, self.metrics, self.cuda_graph)
+        pairs = (([dense, sparse], labels) for dense, sparse, labels in batches)
+        return self._evaluator.run(self.model, pairs, lambda inputs: self._setup(inputs[0]))

@@ -51,7 +51,7 @@ def dot_interact(x: torch.Tensor, pad_to: int = 1) -> torch.Tensor:
 
 class _EmbedDotFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, tset: EmbeddingTables, ids, field_table, pad_to, dense, *weights):
+    def forward(ctx, tset: EmbeddingTables, ids, field_table, pad_to, prepare, dense, *weights):
         L.require_cuda(ids, "embed_dot(ids)")
         dense = dense.contiguous()
         B, F = ids.shape
@@ -72,9 +72,7 @@ class _EmbedDotFn(torch.autograd.Function):
         ctx.tset, ctx.ids, ctx.field_table = tset, ids, field_table
         # the id-only half of K2 (keys, sort, segments) starts now on a side stream and hides
         # behind the top MLP; the backward then only runs the gradient-dependent half
-        ctx.prepared = None
-        if tset.optimizer is not None and any(ctx.needs_input_grad):
-            ctx.prepared = tset.prepare_backward(ids, field_table)
+        ctx.prepared = tset.prepare_backward(ids, field_table) if prepare else None
         ctx.save_for_backward(dense)
         return out
 
@@ -105,9 +103,9 @@ class _EmbedDotFn(torch.autograd.Function):
                 tset.apply_prepared_async(ctx.prepared, gemb)
             else:
                 tset.apply_prepared(ctx.prepared, gemb)
-            return (None, None, None, None, gdense) + (None,) * len(wl)
+            return (None, None, None, None, None, gdense) + (None,) * len(wl)
         wgrads = tset.grads_from_lookup_grad(ids, field_table, gemb, "BF", None)
-        return (None, None, None, None, gdense) + wgrads
+        return (None, None, None, None, None, gdense) + wgrads
 
 
 def embed_dot(tset: EmbeddingTables, ids: torch.Tensor, dense: torch.Tensor,
@@ -120,4 +118,10 @@ def embed_dot(tset: EmbeddingTables, ids: torch.Tensor, dense: torch.Tensor,
     if field_table is None:
         field_table = tuple(range(len(wl)))
     tset.wait_pending()
-    return _EmbedDotFn.apply(tset, ids, tuple(field_table), pad_to, dense, *wl)
+    # K2's id-only half is prepared only when a backward can follow.  ctx.needs_input_grad cannot
+    # decide this: it stays True for the table Parameters inside torch.no_grad(), and
+    # torch.is_grad_enabled() is always False inside Function.forward.  Under grad mode this is
+    # exactly `any(ctx.needs_input_grad)` (ids are integers, never differentiable).
+    prepare = (tset.optimizer is not None and torch.is_grad_enabled()
+               and (dense.requires_grad or any(w.requires_grad for w in wl)))
+    return _EmbedDotFn.apply(tset, ids, tuple(field_table), pad_to, prepare, dense, *wl)

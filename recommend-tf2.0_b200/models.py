@@ -277,17 +277,21 @@ class Trainer:
     for any model of this module: embedding tables are updated in place by K2's fused sparse
     Adam during the backward, every other parameter by one rtf_dense_adam launch (Keras form).
 
-        tr = Trainer(model, loss_fn)          # loss_fn(outputs, labels) -> scalar tensor
-        loss = tr.step(inputs, labels)
+        tr = Trainer(model, loss_fn, metrics=[AUC()])   # loss_fn(outputs, labels) -> scalar
+        loss = tr.step(inputs, labels)        # also updates tr.metrics (inside the graph too)
+        tr.evaluate([(inputs, labels), ...])  # {"loss": ..., "auc": ...}, Keras model.evaluate
 
     The lazily built layers are created by a no-grad eval forward on the first batch (BatchNorm
     moving statistics and the tables do not move)."""
 
     def __init__(self, model: Layer, loss_fn, lr: float = 1e-3, embed_l2: float = 0.0,
-                 cuda_graph: bool = False):
+                 cuda_graph: bool = False, metrics=None):
         from .core import DenseAdam, StepGraph
         self._DenseAdam = DenseAdam
         self.model, self.loss_fn, self.lr = model, loss_fn, lr
+        self.metrics = list(metrics or [])
+        self.cuda_graph = cuda_graph
+        self._evaluator = None
         self.tables = [m for m in model.modules() if isinstance(m, EmbeddingTables)]
         for ts in self.tables:
             if ts.optimizer is None:
@@ -328,6 +332,8 @@ class Trainer:
     def _body(self, inputs, labels):
         out = self.model(inputs)
         loss = self.loss_fn(out, labels)
+        for m in self.metrics:
+            m.update_state(labels, out.detach())
         self.dense_opt.zero_grad()
         loss.backward()
         self.dense_opt.apply()
@@ -342,3 +348,23 @@ class Trainer:
             return self.graph(inputs, labels)
         self._advance()
         return self._body(inputs, labels)
+
+    def _eval_forward(self, inputs, labels):
+        out = self.model(inputs)
+        return out, self.loss_fn(out, labels)
+
+    def evaluate(self, batches) -> dict:
+        """Keras `model.evaluate` over `(inputs, labels)` pairs: the mean loss (weighted by batch
+        size) and every metric of the trainer, computed by fresh copies of the metrics.  Changes
+        no parameter, buffer, table, optimizer state or step counter (metrics.Evaluator)."""
+        if isinstance(self.model, YoutubeDNN):
+            raise TypeError("Trainer.evaluate: YoutubeDNN's forward advances its sampler seed; "
+                            "matching models are not evaluated here")
+        if self._evaluator is None:
+            from .metrics import Evaluator
+            self._evaluator = Evaluator(self._eval_forward, self.metrics, self.cuda_graph)
+
+        def prepare(inputs):
+            if self.dense_opt is None:      # build the layers and flatten before any capture
+                self._setup(inputs)
+        return self._evaluator.run(self.model, batches, prepare)
