@@ -430,6 +430,37 @@ int rtf_dense_gemm_tn(const float* d_a, int64_t lda, int64_t stride_a, const flo
                       int64_t stride_d, int M, int N, int K, int batch, void* d_ws, size_t ws_bytes,
                       void* stream);
 
+/* The same GEMMs fed operands already split into three bf16 planes (csrc/dense_gemm_planes.cuh):
+ * no transform warps in the mainloop, and the output is bit-identical to the fp32 entry points'
+ * for the planes rtf_split_bf16x3 makes of their operands.  An operand is one bf16 tensor of
+ * three planes: plane p of the element the fp32 entry point reads at offset o sits at
+ * p * plane_* + o.  Strides, leading dimensions and plane strides % 8 == 0 (16 bytes) for the
+ * planes, % 4 for the output; pointers 16-byte aligned; else RTF_E_ALIGN.
+ *
+ * rtf_split_bf16x3: planes[p * plane_stride + r * ld_out + c] = plane p of x[r * ld_in + c]:
+ *   x0 = RN_satfinite(x), r = (x - x0) * 2^8, x1 = RN_satfinite(r), x2 = RN_satfinite((r - x1) * 2^8)
+ *   (bf16; the GEMM mainloop's own split).  cols, ld_in, ld_out, plane_stride even.           */
+int rtf_split_bf16x3(const float* d_x, int64_t rows, int cols, int64_t ld_in, uint16_t* d_planes,
+                     int64_t ld_out, int64_t plane_stride, void* stream);
+int rtf_dense_gemm_nn_planes_workspace(int M, int N, int K, int batch, size_t* bytes);
+int rtf_dense_gemm_nt_planes_workspace(int M, int N, int K, int batch, size_t* bytes);
+int rtf_dense_gemm_tn_planes_workspace(int M, int N, int K, int batch, size_t* bytes);
+int rtf_dense_gemm_nn_planes(const uint16_t* d_a, int64_t lda, int64_t stride_a, int64_t plane_a,
+                             const uint16_t* d_b, int64_t ldb, int64_t stride_b, int64_t plane_b,
+                             const float* d_bias, int relu, float* d_out, int64_t ldd,
+                             int64_t stride_d, int M, int N, int K, int batch, void* d_ws,
+                             size_t ws_bytes, void* stream);
+int rtf_dense_gemm_nt_planes(const uint16_t* d_a, int64_t lda, int64_t stride_a, int64_t plane_a,
+                             const uint16_t* d_b, int64_t ldb, int64_t stride_b, int64_t plane_b,
+                             const float* d_bias, int relu, float* d_out, int64_t ldd,
+                             int64_t stride_d, int M, int N, int K, int batch, void* d_ws,
+                             size_t ws_bytes, void* stream);
+int rtf_dense_gemm_tn_planes(const uint16_t* d_a, int64_t lda, int64_t stride_a, int64_t plane_a,
+                             const uint16_t* d_b, int64_t ldb, int64_t stride_b, int64_t plane_b,
+                             const float* d_bias, int relu, float* d_out, int64_t ldd,
+                             int64_t stride_d, int M, int N, int K, int batch, void* d_ws,
+                             size_t ws_bytes, void* stream);
+
 /* ---- K6: AutoInt interacting layer, fused ---------------------------------------------------
  * replaces: ctr.layers.modules.MultiHeadAttention.call on a self-attention input X (B, F, dm):
  *           Q,K,V = act(X W{q,k,v}) (no bias, src/ctr/layers/modules.py:255-270), per-head

@@ -104,6 +104,16 @@ SIGNATURES = {
                           _int, _p, C.c_size_t, _p],
     "rtf_dense_gemm_tn": [_p, _i64, _i64, _p, _i64, _i64, _p, _int, _p, _i64, _i64, _int, _int, _int,
                           _int, _p, C.c_size_t, _p],
+    "rtf_split_bf16x3": [_p, _i64, _int, _i64, _p, _i64, _i64, _p],
+    "rtf_dense_gemm_nn_planes_workspace": [_int, _int, _int, _int, C.POINTER(C.c_size_t)],
+    "rtf_dense_gemm_nt_planes_workspace": [_int, _int, _int, _int, C.POINTER(C.c_size_t)],
+    "rtf_dense_gemm_tn_planes_workspace": [_int, _int, _int, _int, C.POINTER(C.c_size_t)],
+    "rtf_dense_gemm_nn_planes": [_p, _i64, _i64, _i64, _p, _i64, _i64, _i64, _p, _int, _p, _i64, _i64,
+                                 _int, _int, _int, _int, _p, C.c_size_t, _p],
+    "rtf_dense_gemm_nt_planes": [_p, _i64, _i64, _i64, _p, _i64, _i64, _i64, _p, _int, _p, _i64, _i64,
+                                 _int, _int, _int, _int, _p, C.c_size_t, _p],
+    "rtf_dense_gemm_tn_planes": [_p, _i64, _i64, _i64, _p, _i64, _i64, _i64, _p, _int, _p, _i64, _i64,
+                                 _int, _int, _int, _int, _p, C.c_size_t, _p],
     "rtf_fm_layer_workspace": [_i64, _int, C.POINTER(C.c_size_t)],
     "rtf_fm_layer_fwd": [_p, _i64, _p, _int, _p, _i64, _int, _int, _i64, _int, _int, _p, _p, _p],
     "rtf_fm_layer_bwd": [_p, _i64, _p, _int, _p, _i64, _int, _int, _i64, _int, _int, _p, _p,

@@ -164,6 +164,24 @@ def set_dense_gemm(kind: str) -> None:
     DENSE_GEMM = kind
 
 
+# bf16x6 layers large enough to repay splitting their operands into bf16 planes once (a pass at
+# HBM rate per operand, 10 B per value) run the plane-fed GEMM (csrc/dense_gemm_planes.cuh), whose
+# mainloop has no transform warps; the results are bit-identical to the fp32-fed GEMM.  Measured
+# on a B200 at B = 65 536 (profiles/r4_dense_planes.jsonl), the saving beats the split passes when
+# K N / (K + N) >= 256: the 480-1024-1024-512 layers of the DLRM top MLP, not its 512-256 or
+# the bottom MLP's 512-256-128 layers.  set_dense_planes(False) forces the fp32-fed GEMM.
+DENSE_PLANES = True
+
+
+def set_dense_planes(on: bool) -> None:
+    global DENSE_PLANES
+    DENSE_PLANES = bool(on)
+
+
+def _planes_pay(M: int, K: int, N: int) -> bool:
+    return DENSE_PLANES and K % 8 == 0 and N % 8 == 0 and K * N >= 256 * (K + N)
+
+
 def _x6_ok(*mats) -> bool:
     if DENSE_GEMM != "bf16x6":
         return False
@@ -211,6 +229,64 @@ def dense_gemm(kind: str, a: torch.Tensor, b: torch.Tensor, bias=None, relu: boo
             int(relu), out.data_ptr(), N, sd, M, N, K, batch, ws.data_ptr(), ws.numel(),
             L.current_stream_ptr())
     L.check(rc, f"rtf_dense_gemm_{kind}")
+    return out.sum(0) if batch > 1 else out
+
+
+def split_planes(x: torch.Tensor) -> torch.Tensor:
+    """Split a contiguous 2-D fp32 CUDA tensor (R, C) into its three bf16 planes, a (3, R, C)
+    bf16 tensor with x ~= p0 + p1 * 2^-8 + p2 * 2^-16: the operand split the dense GEMM's
+    mainloop makes (rtf_split_bf16x3)."""
+    from . import _lib as L
+    if not (x.is_cuda and x.dtype == torch.float32 and x.dim() == 2 and x.is_contiguous()):
+        raise ValueError("split_planes takes a contiguous 2-D fp32 CUDA tensor")
+    R, Cc = x.shape
+    p = torch.empty((3, R, Cc), dtype=torch.bfloat16, device=x.device)
+    L.check(L.lib().rtf_split_bf16x3(x.data_ptr(), R, Cc, Cc, p.data_ptr(), Cc, R * Cc,
+                                     L.current_stream_ptr()), "rtf_split_bf16x3")
+    return p
+
+
+def dense_gemm_planes(kind: str, a: torch.Tensor, b: torch.Tensor, bias=None, relu: bool = False,
+                      splits: int = 1) -> torch.Tensor:
+    """dense_gemm on operands given as bf16 planes (split_planes): a, b are (3, rows, cols)
+    contiguous bf16 tensors holding the planes of the 2-D fp32 operands dense_gemm takes.  The
+    result is bit-identical to dense_gemm on the fp32 operands the planes were split from."""
+    import ctypes as C
+    from . import _lib as L
+    lib = L.lib()
+    for m in (a, b):
+        if not (m.is_cuda and m.dtype == torch.bfloat16 and m.dim() == 3 and m.shape[0] == 3
+                and m.is_contiguous()):
+            raise ValueError("plane operands are contiguous (3, rows, cols) bf16 CUDA tensors")
+    if kind == "nn":
+        (M, K), N = a.shape[1:], b.shape[2]
+    elif kind == "nt":
+        (M, K), N = a.shape[1:], b.shape[1]
+    elif kind == "tn":
+        (K, M), N = a.shape[1:], b.shape[2]
+    else:
+        raise ValueError(kind)
+    fn = getattr(lib, f"rtf_dense_gemm_{kind}_planes")
+    wsq = getattr(lib, f"rtf_dense_gemm_{kind}_planes_workspace")
+    lda, ldb = a.stride(1), b.stride(1)
+    sa = sb = sd = 0
+    batch = 1
+    if kind == "tn" and splits > 1:
+        if K % splits or (K // splits) % 4:
+            raise ValueError("splits must divide K into multiples of 4")
+        batch, K = splits, K // splits
+        sa, sb, sd = K * lda, K * ldb, M * N
+    out = torch.empty((batch, M, N) if batch > 1 else (M, N), dtype=torch.float32, device=a.device)
+    key = (kind + "_planes", M, N, K, batch)
+    if key not in _GEMM_WS_BYTES:
+        nb = C.c_size_t(0)
+        L.check(wsq(M, N, K, batch, C.byref(nb)), f"rtf_dense_gemm_{kind}_planes_workspace")
+        _GEMM_WS_BYTES[key] = max(nb.value, 16)
+    ws = _scratch(_GEMM_WS_BYTES[key], a.device)
+    rc = fn(a.data_ptr(), lda, sa, a.stride(0), b.data_ptr(), ldb, sb, b.stride(0),
+            None if bias is None else bias.data_ptr(), int(relu), out.data_ptr(), N, sd, M, N, K,
+            batch, ws.data_ptr(), ws.numel(), L.current_stream_ptr())
+    L.check(rc, f"rtf_dense_gemm_{kind}_planes")
     return out.sum(0) if batch > 1 else out
 
 
@@ -299,7 +375,16 @@ class _DenseFn(torch.autograd.Function):
             x = F.pad(x, (0, kpad))
             w = F.pad(w, (0, 0, 0, kpad))
         ctx.kpad = kpad
+        ctx.planes = False
         if x.shape[0] >= 1024 and _x6_ok(x, w) and b.data_ptr() % 16 == 0:
+            if _planes_pay(*x.shape, w.shape[1]):
+                # split x and W into bf16 planes once; the backward's dgrad and wgrad reuse them
+                ctx.planes = True
+                xp, wp = split_planes(x), split_planes(w)
+                y = dense_gemm_planes("nn", xp, wp, b, relu)
+                ctx.save_for_backward(xp, wp, y if relu else None)
+                ctx.relu = relu
+                return y
             y = dense_gemm("nn", x, w, b, relu)
         else:
             y = torch._addmm_activation(b, x, w, use_gelu=False) if relu else torch.addmm(b, x, w)
@@ -311,6 +396,17 @@ class _DenseFn(torch.autograd.Function):
     def backward(ctx, gy):
         x, w, y = ctx.saved_tensors
         g, gb = _relu_bwd_bias_grad(gy, y if ctx.relu else None)
+        if ctx.planes:   # x, w are the planes of the forward's operands
+            gp = split_planes(g)
+            gx = dense_gemm_planes("nt", gp, w) if ctx.needs_input_grad[0] else None
+            gw = None
+            if ctx.needs_input_grad[1]:
+                B = g.shape[0]
+                gw = dense_gemm_planes("tn", x, gp, splits=_wgrad_splits(B, x.shape[2], g.shape[1]))
+            if ctx.kpad:   # the K padding of the forward (e.g. a 479-wide interaction -> 480)
+                gx = None if gx is None else gx[:, : gx.shape[1] - ctx.kpad].contiguous()
+                gw = None if gw is None else gw[: gw.shape[0] - ctx.kpad]
+            return gx, gw, gb, None
         gx = None
         if ctx.needs_input_grad[0]:
             gx = dense_gemm("nt", g, w) if (g.shape[0] >= 1024 and _x6_ok(g, w)) else g @ w.t()

@@ -37,6 +37,7 @@
 #include "cutlass/numeric_types.h"
 
 #include "rtf_b200.h"
+#include "dense_gemm_planes.cuh"
 
 namespace rtf_gemm {
 
@@ -148,7 +149,116 @@ struct FastF32Gemm {
     if (Gemm::get_workspace_size(args) > ws_bytes) return RTF_E_WORKSPACE;
     if (gemm.initialize(args, ws, st) != cutlass::Status::kSuccess) return RTF_E_ARG;
     cutlass::Status s = gemm.run(st);
-    if (s != cutlass::Status::kSuccess) return (int)cudaGetLastError() ? (int)cudaGetLastError() : RTF_E_ARG;
+    if (s != cutlass::Status::kSuccess) {
+      const int e = (int)cudaGetLastError();  // read once: the call clears a non-sticky error
+      return e ? e : RTF_E_ARG;
+    }
+    return 0;
+  }
+};
+
+// The same GEMM fed pre-split bf16 planes (dense_gemm_planes.cuh): same tile, cluster, TiledMma
+// (band order, ScalingFactor), promotion interval, accumulator stages and epilogue as
+// FastF32Gemm, so D is bit-identical to FastF32Gemm's for the planes its transform would make.
+// A[l] planes: bf16 at pa + p * pstride_a + <the fp32 operand's offset>, p = 0, 1, 2.
+template <class LayoutA, class LayoutB, int Bands, int PromotionInterval = 2>
+struct FastF32PlanesGemm {
+  using Ref = FastF32Gemm<LayoutA, LayoutB, Bands>;
+  using Epilogue = typename Ref::Epilogue;
+  using SP = typename Ref::SP;
+  using Stock = typename Ref::Stock;
+  static constexpr bool a_k = std::is_same_v<LayoutA, RowMajor>;
+  static constexpr bool b_k = std::is_same_v<LayoutB, ColumnMajor>;
+  using StrideA = PlaneStride<a_k>;
+  using StrideB = PlaneStride<b_k>;
+  using TileShape = typename Stock::TileShape;
+  using TiledMma = typename Stock::TiledMma;
+  using AtomA = typename Stock::SmemLayoutAtomsA::ComputeLayoutAtom;
+  using AtomB = typename Stock::SmemLayoutAtomsB::ComputeLayoutAtom;
+  // bytes of one pipeline stage in one CTA: three bf16 planes of the A and B k-blocks
+  static constexpr int kStageBytes =
+      3 * 2 * (size<0>(TileShape{}) / 2 + size<1>(TileShape{}) / 2) * size<2>(TileShape{});
+  static constexpr int kStages =
+      (cutlass::arch::sm100_smem_capacity_bytes - static_cast<int>(sizeof(typename Epilogue::SharedStorage)) -
+       4096) / kStageBytes;
+  using Policy = MainloopSm100FastF32Planes<kStages, SP::Schedule::SchedulerPipelineStageCount,
+                                            SP::Schedule::AccumulatorPipelineStageCount, Bands,
+                                            SP::ScalingFactor, PromotionInterval, typename SP::ClusterShape>;
+  using Mainloop = cutlass::gemm::collective::CollectiveMma<
+      Policy, TileShape, cutlass::bfloat16_t, StrideA, cutlass::bfloat16_t, StrideB, TiledMma,
+      cute::SM100_TMA_2SM_LOAD, AtomA, void, cute::identity, cute::SM100_TMA_2SM_LOAD, AtomB, void,
+      cute::identity>;
+  using Kernel = cutlass::gemm::kernel::GemmUniversal<Shape<int, int, int, int>, Mainloop, Epilogue>;
+  using Gemm = cutlass::gemm::device::GemmUniversalAdapter<Kernel>;
+  using StrideD = typename Kernel::StrideD;
+
+  template <class Stride, bool KContiguous>
+  static Stride make_stride(int64_t ld, int64_t batch, int64_t plane) {
+    Stride s{};
+    if constexpr (KContiguous) {
+      get<0>(s) = ld;
+    } else {
+      get<1>(s) = ld;
+    }
+    get<2, 0>(s) = plane;
+    get<2, 1>(s) = batch;
+    return s;
+  }
+
+  static typename Gemm::Arguments make_args(const uint16_t* A, int64_t lda, int64_t sA, int64_t pA,
+                                            const uint16_t* B, int64_t ldb, int64_t sB, int64_t pB,
+                                            const float* bias, float lo, float hi, float* D,
+                                            int64_t ldd, int64_t sD, int M, int N, int K, int batch) {
+    StrideD sd = Ref::template make_stride<StrideD, true>(ldd, sD);
+    typename Gemm::Arguments args{cutlass::gemm::GemmUniversalMode::kGemm,
+                                  {M, N, K, batch},
+                                  {reinterpret_cast<const cutlass::bfloat16_t*>(A),
+                                   make_stride<StrideA, a_k>(lda, sA, pA),
+                                   reinterpret_cast<const cutlass::bfloat16_t*>(B),
+                                   make_stride<StrideB, b_k>(ldb, sB, pB)},
+                                  {{}, nullptr, sd, D, sd}};
+    args.epilogue.thread.alpha = 1.f;
+    args.epilogue.thread.beta = 0.f;
+    args.epilogue.thread.bias_ptr = bias;
+    args.epilogue.thread.activation.lower_bound = lo;
+    args.epilogue.thread.activation.upper_bound = hi;
+    static int sm_count = 0;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (sm_count == 0) cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
+    args.hw_info.device_id = dev;
+    args.hw_info.sm_count = sm_count;
+    return args;
+  }
+
+  static int workspace(int M, int N, int K, int batch, size_t* bytes) {
+    auto args = make_args(nullptr, K, 0, 0, nullptr, K, 0, 0, nullptr, 0.f, 0.f, nullptr, N, 0, M,
+                          N, K, batch);
+    *bytes = Gemm::get_workspace_size(args);
+    return 0;
+  }
+
+  // bf16 TMA: 16-byte aligned bases and strides, i.e. every stride a multiple of 8 elements
+  static int run(const uint16_t* A, int64_t lda, int64_t sA, int64_t pA, const uint16_t* B,
+                 int64_t ldb, int64_t sB, int64_t pB, const float* bias, int relu, float* D,
+                 int64_t ldd, int64_t sD, int M, int N, int K, int batch, void* ws, size_t ws_bytes,
+                 cudaStream_t st) {
+    if (!A || !B || !D || M <= 0 || N <= 0 || K <= 0 || batch <= 0 || pA <= 0 || pB <= 0)
+      return RTF_E_ARG;
+    if (lda % 8 || ldb % 8 || sA % 8 || sB % 8 || pA % 8 || pB % 8 || ldd % 4 || sD % 4 ||
+        (uintptr_t)A % 16 || (uintptr_t)B % 16 || (uintptr_t)D % 16 || (uintptr_t)bias % 16)
+      return RTF_E_ALIGN;
+    const float lo = relu ? 0.f : -INFINITY, hi = INFINITY;
+    auto args = make_args(A, lda, sA, pA, B, ldb, sB, pB, bias, lo, hi, D, ldd, sD, M, N, K, batch);
+    Gemm gemm;
+    if (gemm.can_implement(args) != cutlass::Status::kSuccess) return RTF_E_RANGE;
+    if (Gemm::get_workspace_size(args) > ws_bytes) return RTF_E_WORKSPACE;
+    if (gemm.initialize(args, ws, st) != cutlass::Status::kSuccess) return RTF_E_ARG;
+    cutlass::Status s = gemm.run(st);
+    if (s != cutlass::Status::kSuccess) {
+      const int e = (int)cudaGetLastError();  // read once: the call clears a non-sticky error
+      return e ? e : RTF_E_ARG;
+    }
     return 0;
   }
 };

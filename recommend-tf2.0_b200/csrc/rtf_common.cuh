@@ -94,6 +94,29 @@ __device__ __forceinline__ void bulk_g2s(void* smem_dst, const void* gmem_src, u
       : "memory");
 }
 
+// ---- fp32 -> three bf16 planes (the dense GEMM's operand split) -------------------
+// The transform of CUTLASS's emulated FastF32 mainloop, restated bit for bit, for a pair of
+// values (a, b) -> bf16x2 words {lo = a, hi = b}:
+//   x0 = RN_satfinite(x);  r = (x - x0) * 2^S;  x1 = RN_satfinite(r);  x2 = RN_satfinite((r - x1) * 2^S)
+// S = kPlaneScale is the mainloop's ScalingFactor (8 for bf16).
+constexpr int kPlaneScale = 8;
+__device__ __forceinline__ uint32_t cvt_bf16x2_satfinite(float lo, float hi) {
+  uint32_t d;
+  asm("cvt.rn.satfinite.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
+  return d;
+}
+__device__ __forceinline__ void split_bf16x3(float a, float b, uint32_t& p0, uint32_t& p1,
+                                             uint32_t& p2) {
+  const float s = (float)(1 << kPlaneScale);
+  p0 = cvt_bf16x2_satfinite(a, b);
+  a = __fmul_rn(__fsub_rn(a, __uint_as_float(p0 << 16)), s);
+  b = __fmul_rn(__fsub_rn(b, __uint_as_float(p0 & 0xffff0000u)), s);
+  p1 = cvt_bf16x2_satfinite(a, b);
+  a = __fmul_rn(__fsub_rn(a, __uint_as_float(p1 << 16)), s);
+  b = __fmul_rn(__fsub_rn(b, __uint_as_float(p1 & 0xffff0000u)), s);
+  p2 = cvt_bf16x2_satfinite(a, b);
+}
+
 // id load with bounds check; returns -1 for an out-of-range id
 template <typename IdT>
 __device__ __forceinline__ long long load_id(const IdT* ids, long long idx, long long rows,
